@@ -14,6 +14,8 @@ checksum of (ref, query, ani, af_ref, af_query) are all-reduced over the ranks (
 sample of kept pairs is re-chained by the CPU oracle (1e-4).  With N > 1 (or --shuffle-order) the whole measurement is
 repeated on a seeded random permutation of the genome order (input order unrelated to relatedness: the worst case of the
 multi-GPU exchange) and reported under "shuffled".
+`--dump-outputs DIR` writes the kept pairs of the last timed step of the headline leg to DIR/<field>.npy (see dump_outputs),
+so that two builds run with the same arguments can be compared output for output.
 `--impl reference` times the reference's CPU algorithm (the C++ restatement in oracle/: the Rust crate cannot be built
 in this image) on all host cores on the SAME configuration (full genome set).
 """
@@ -64,6 +66,8 @@ def parse():
     ap.add_argument("--no-shuffle", action="store_true", help="skip the permuted-order measurement (A/B sessions)")
     ap.add_argument("--perm-seed", type=int, default=12345)
     ap.add_argument("--spot-check", type=int, default=200, help="kept pairs re-chained by the CPU oracle after the timed legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<field>.npy (rows sorted by ref_id, query_id)")
     a = ap.parse_args()
     cfg = dict(CONFIGS[a.config])
     for k in ("genomes", "genome_len", "cluster"):
@@ -238,15 +242,11 @@ def run_reference(args):
     N = args.genomes
     total_pairs = N * (N - 1) // 2
     runs = []
-    warm, steps = args.warmup, args.steps
-    i = 0
-    while i < warm + steps:
+    warm = args.warmup
+    for i in range(warm + args.steps):
         d = cpu_triangle(O, cfg, N, threads)
-        if i == 0 and d["t_total"] > 30:   # one step already takes longer than the 30 s budget: no warm-up, at most 2 steps
-            warm, steps = 0, min(steps, 2)
         if i >= warm:
             runs.append(d)
-        i += 1
     t = float(np.mean([r["t_total"] for r in runs]))
     v = total_pairs / t
     last = runs[-1]
@@ -322,6 +322,35 @@ def oracle_spot_check(res, ids, cfg, n_sample, seed):
         for f in ("ani", "af_ref", "af_query"):
             worst = max(worst, abs(float(r[f]) - float(getattr(o, f))))
     return {"pairs": int(len(pick)), "max_abs_diff": worst, "tolerance": 1e-4, "ok": bool(worst <= 1e-4)}
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def pair_key(res):
+    """64-bit mix of (ref_id, query_id): a fixed pseudo-random order of the pairs, the same whichever build computed them."""
+    u64 = np.uint64
+    with np.errstate(over="ignore"):
+        x = ((res["ref_id"].astype(u64) << u64(32)) | res["query_id"].astype(u64)) * u64(0x9E3779B97F4A7C15)
+        x ^= x >> u64(31)
+        return x * u64(0xD6E8FEB86659FD93)
+
+
+def dump_outputs(res, out_dir):
+    """One DIR/<field>.npy per RESULT_DTYPE field of the kept pairs, rows sorted by (ref_id, query_id): scores in float32 as
+    computed, ids and counts in float64 (exact).  When all rows would exceed 64 MB, the pairs with the smallest pair_key
+    are written, so that two builds sample the same pairs."""
+    cols = [(n, np.float32 if res.dtype[n] == np.float32 else np.float64) for n in res.dtype.names]
+    row_bytes = sum(np.dtype(t).itemsize for _, t in cols)
+    n_max = (DUMP_LIMIT - (1 << 20)) // row_bytes          # 1 MB left for the .npy headers
+    sampled = len(res) > n_max
+    if sampled:
+        res = res[np.argsort(pair_key(res), kind="stable")[:n_max]]
+    res = res[np.lexsort((res["query_id"], res["ref_id"]))]
+    os.makedirs(out_dir, exist_ok=True)
+    for n, t in cols:
+        np.save(os.path.join(out_dir, n + ".npy"), res[n].astype(t))
+    return {"dir": out_dir, "rows": int(len(res)), "sampled": sampled}
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -437,6 +466,15 @@ def main():
             step(False)
         ms_val, _, launches = timed(False, args.steps)
         ck_val = allreduce_count_checksum(len(last["res"]), result_checksum(last["res"]), world)
+        dumped = None
+        if args.dump_outputs and order == "contiguous":
+            res = last["res"]
+            if world > 1:
+                parts = [None] * world
+                torch.distributed.all_gather_object(parts, res)
+                res = np.concatenate(parts)
+            if rank == 0:
+                dumped = dump_outputs(res, args.dump_outputs)
         roof = roof_chain = None
         if rank == 0 and order == "contiguous":
             roof = measure_hashpass(ctx, dev_bases, off, goc, nloc, sp, L)
@@ -494,7 +532,7 @@ def main():
                 "verify": {"kept_pairs_all_ranks": ck_e2e[0], "kept_pairs_expected": expected, "kept_ok": ck_e2e[0] == expected == ck_val[0],
                            "checksum_e2e": "%016x" % ck_e2e[1], "checksum_value_leg": "%016x" % ck_val[1],
                            "legs_agree": ck_e2e == ck_val, "oracle_spot_check": spot},
-                "roof": roof, "roof_chain": roof_chain}
+                "roof": roof, "roof_chain": roof_chain, "dumped": dumped}
 
     if rank == 0:
         clocks.start()
@@ -521,6 +559,8 @@ def main():
                         "note": "inputs = ASCII in pinned host memory; host_pack_share of the bases is converted to 2-bit on the host "
                                 "cores inside the timed call (0.25 B/base on the wire), the rest crosses PCIe as ASCII"},
                 "gpu_launches": m["launches"], "clocks": clk, "roofline": m["roof"], "roofline_chain": m["roof_chain"], "cpu_baseline": cpu}
+        if m["dumped"]:
+            line["dumped_outputs"] = m["dumped"]
         if m.get("e2e_2bit_ms_per_step"):
             line["e2e_2bit"] = {"what": "the same call on genomes that are already 2-bit packed in pinned host memory (sk_triangle_2bit; SURVEY 8(d): "
                                         "'resident in host memory as ASCII/2-bit'); results on the host; the ASCII leg above stays the headline `e2e`",
@@ -628,4 +668,5 @@ def measure_chain(ctx, dev_bases, off, goc, nloc, sp, mp, L, G):
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True   # the tree may be read-only: the modules main() imports from it leave no bytecode there
     sys.exit(main())

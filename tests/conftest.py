@@ -6,7 +6,8 @@ import pytest
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
-REF_TEST_FILES = "/root/reference/test_files"
+# skani's own test_files/ directory: the full-size genomes a few oracle golden tests read (too large for tests/golden)
+REF_TEST_FILES = os.environ.get("SKANI_TEST_FILES", "")
 
 
 def pytest_configure(config):
@@ -15,11 +16,11 @@ def pytest_configure(config):
 
 
 def have_reference():
-    return os.path.isdir(REF_TEST_FILES)
+    return bool(REF_TEST_FILES) and os.path.isdir(REF_TEST_FILES)
 
 
 needs_reference = pytest.mark.skipif(not have_reference(),
-                                     reason="/root/reference fixtures not present (GPU box)")
+                                     reason="needs SKANI_TEST_FILES = skani's test_files directory (full-size genomes)")
 
 
 def db_tool():

@@ -1,7 +1,10 @@
 """ctypes binding of the CPU oracle (oracle/liboracle.so).  TEST INFRASTRUCTURE ONLY."""
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -35,10 +38,13 @@ def build():
 
 
 def build_native():
-    """-march=native build for the CPU baseline (oracle/_native/liboracle.so); returns its path or None."""
+    """-march=native build for the CPU baseline, made in a new temporary directory (the tree may be read-only) that is
+    removed at exit; returns the library's path or None."""
     try:
-        subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "native"])
-        return os.path.join(ORACLE_DIR, "_native", "liboracle.so")
+        d = tempfile.mkdtemp(prefix="skani-oracle-native-")
+        atexit.register(shutil.rmtree, d, True)
+        subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "native", "NATIVE_DIR=" + d])
+        return os.path.join(d, "liboracle.so")
     except Exception:
         return None
 
